@@ -2,7 +2,7 @@
 bench.py -- anomaly windows/sec of the fused predict+score hot path on BASELINE.json configs[1]:
 1 000 machines x 64-tag feedforward_hourglass autoencoder, 10 000 rows per machine, per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--machines M] [--rows R] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--machines M] [--rows R] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one pass of the hot path (gb_ffae_infer_score) over every machine of the rank: 10^7 windows per GPU, inputs
@@ -39,6 +39,7 @@ BYTES_PER_WINDOW = 4 * T + 4 * T + 4 * 4 * T + 12  # read x, y; write model-outp
 # dram__bytes_read.sum + dram__bytes_write.sum per window from the committed `ncu --set full` captures (profiles/, file names below)
 NCU_DRAM_BYTES_PER_WINDOW = {"tcgen05": (1.569383e9 + 3.048933e9) / 3.0e6, "fma": (1.037003e9 + 2.019607e9) / 2.0e6}
 NCU_SOURCE = {"tcgen05": "profiles/r02_ffae_tc_ncu.txt (300-machine capture)", "fma": "profiles/r01_ffae_infer_fma_ncu.txt (200-machine capture)"}
+DUMP_BYTES = 32 << 20  # --dump-outputs: a seeded sample of rows of every output, this many bytes in all
 METRIC = "anomaly windows/sec (64-tag feedforward_hourglass AE, 1k machines x 10k rows per GPU, fused predict+score)"
 
 
@@ -251,6 +252,21 @@ def workload_config(machines, rows, world, variant=None):
 
 
 # ------------------------------------------------------------------------------------------------ GPU arm
+def dump_outputs(out, total_rows, dest):
+    """
+    Writes what a caller of the hot path receives (every output array of one step) as <dest>/<name>.npy, float32, on the same
+    seeded sample of rows for every array and every run, so that the outputs of two builds can be compared array by array.
+    """
+    import torch
+
+    os.makedirs(dest, exist_ok=True)
+    per_row = sum(t[0].numel() * t.element_size() for t in out.values())
+    rows = np.sort(np.random.default_rng(0).choice(total_rows, size=min(total_rows, DUMP_BYTES // per_row), replace=False))
+    idx = torch.from_numpy(rows).to(next(iter(out.values())).device)
+    for name, t in out.items():
+        np.save(os.path.join(dest, f"{name}.npy"), t.index_select(0, idx).cpu().numpy())
+
+
 _REAL_STDOUT = None
 
 
@@ -282,6 +298,7 @@ def main():
     ap.add_argument("--cpu-machines", type=int, default=150, help="machines in the one-core cpu_baseline sample (~10 s of CPU work)")
     ap.add_argument("--secondary", type=int, default=1, help="0: skip the configs[2]/[3]/[4] block")
     ap.add_argument("--numa", type=int, default=1, help="0: do not bind the rank to its GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rank 0's outputs of the last timed step (a fixed sample of rows) to DIR/<name>.npy")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -289,6 +306,8 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs needs --impl ours: the reference arm keeps no outputs")
         run_reference_arm(args, rank, world)
         return
 
@@ -349,6 +368,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     elapsed_ms = ev[0].elapsed_time(ev[-1])
     per_launch_ms = [ev[i].elapsed_time(ev[i + 1]) for i in range(args.steps)]
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(out, M * R, args.dump_outputs)
     t = torch.tensor([elapsed_ms], device=dev, dtype=torch.float64)
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

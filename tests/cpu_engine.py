@@ -1,8 +1,8 @@
 """
 TEST INFRASTRUCTURE ONLY.  A CPU stand-in for the compute entry points of ``gordo_components_b200.engine``, built on the
 oracle (``oracle/keras_math.py``, ``oracle/anomaly_math.py``), so that the *host-side* protocol of the estimator classes --
-what gordo's serializer, ModelBuilder and server call on them -- can be exercised end to end in the GPU-less container, with
-the reference's own callers executed from /root/reference (tests/test_reference_dropin.py).
+what gordo's serializer, ModelBuilder and server call on them -- can be exercised end to end without a GPU
+(tests/test_reference_dropin.py, and tests/golden/make_golden.py for its fixture).
 
 The product has no CPU path: this module is never imported by the package, and the numbers it produces are the oracle's, not
 a parity claim about the kernels (those are tests/test_gpu_*.py on a B200).  ``patched_engine()`` swaps the entry points in and

@@ -11,6 +11,11 @@ Fixtures written:
                              block of DiffBasedAnomalyDetector.anomaly() from the reference
   ffnet_anomaly.npz          the same, with the base estimator being a fixed-weight hourglass
                              net (oracle/keras_math.ff_forward): pins net -> anomaly end to end
+  detector_sma_seed<s>.npz   a fitted DiffBasedAnomalyDetector (LinearRegression base, SMA
+                             smoothing): its predictions, thresholds and anomaly frame
+  dropin.{json,npz}          the INTEGRATION.md definition driven through the reference's
+                             from_definition / into_definition / ModelBuilder._build /
+                             serializer, with this package's estimators on the CPU oracle
 """
 from __future__ import annotations
 
@@ -301,6 +306,78 @@ def callers_fixture():
     print("callers ok:", len(out["expansions"]), "expansions;", {k: len(v["build_metadata"]["model"]["cross_validation"]["scores"]) for k, v in out["build"].items()})
 
 
+def detector_fixture(seed):
+    """The reference's DiffBasedAnomalyDetector cross-validated and fitted on random frames (tests/test_oracle_golden.py)."""
+    rng = np.random.default_rng(seed)
+    X = pd.DataFrame(rng.random((240, 5)))
+    y = pd.DataFrame(rng.random((240, 5)) * 3.0)
+    det = ref.DiffBasedAnomalyDetector(base_estimator=MultiOutputRegressor(LinearRegression()), scaler=MinMaxScaler(), window=10, smoothing_method="sma")
+    det.cross_validate(X=X, y=y)
+    det.fit(X, y)
+    frame = det.anomaly(X, y)
+    save = dict(X=X.values, y=y.values, window=10, method="sma", pred=np.asarray(det.predict(X), dtype=np.float64),
+                feature_thresholds=det.feature_thresholds_.values.astype(np.float64), aggregate_threshold=np.float64(det.aggregate_threshold_),
+                hourglass_dims_0p5_3_64=np.array(ref.hourglass_calc_dims(0.5, 3, 64)))
+    for top in dict.fromkeys(frame.columns.get_level_values(0)):
+        if top not in ("start", "end"):
+            save[f"frame_{top}"] = np.asarray(frame[top], dtype=np.float64)
+    np.savez_compressed(os.path.join(HERE, f"detector_sma_seed{seed}.npz"), **save)
+    print(f"detector_sma_seed{seed} ok", frame.shape)
+
+
+def dropin_fixture():
+    """
+    The drop-in definition of tests/test_reference_dropin.py through the reference's own callers: its definition expansion, the
+    build metadata of ModelBuilder._build (this package's estimators computing with the CPU oracle of tests/cpu_engine.py) and the
+    anomaly frame of the model after the reference serializer's dumps/loads.
+    """
+    sys.path.insert(0, os.path.dirname(HERE))
+    from cpu_engine import patched_engine
+    from test_reference_dropin import DEFINITION, EVALUATION, frame, key_tree
+
+    from gordo_components_b200.machine.model import base as b200_base
+    from gordo_components_b200.machine.model.anomaly import base as b200_abase
+    from oracle.reference_loader import load_reference_callers
+
+    rc = load_reference_callers()
+    # gordo only exists once the loader has executed it, so the import-time registration of machine/model/base.py is repeated here
+    assert b200_base.register_with_gordo("gordo.machine.model.base", "GordoBase", b200_base.GordoBase)
+    assert b200_base.register_with_gordo("gordo.machine.model.anomaly.base", "AnomalyDetectorBase", b200_abase.AnomalyDetectorBase)
+    data = frame()
+    expanded = rc.into_definition(rc.from_definition(DEFINITION))
+
+    class Dataset:
+        def get_data(self):
+            return data, data
+
+        def get_metadata(self):
+            return {"rows": len(data)}
+
+    rc.GordoBaseDataset.registry["dropin"] = Dataset()
+    machine = rc.Record(name="dropin-machine", project_name="p", model=DEFINITION, evaluation=dict(EVALUATION), runtime={},
+                        dataset=rc.Record(key="dropin"), metadata=rc.Record(user_defined={}))
+    builder = rc.ModelBuilder.__new__(rc.ModelBuilder)
+    builder.machine, builder.back_compatibles, builder.default_data_provider = machine, None, None
+    with patched_engine():
+        model, built = builder._build()
+        loaded = rc.serializer.loads(rc.serializer.dumps(model))
+        X = data.iloc[-40:]
+        anomaly = loaded.anomaly(X, X, frequency=pd.Timedelta("10min"))
+    mb = built.metadata.build_metadata.to_dict()["model"]
+    tree = key_tree({k: v for k, v in mb.items() if k not in ("model_creation_date", "model_training_duration_sec")})
+    tree["cross_validation"].pop("cv_duration_sec", None)
+    fixture = {"definition": DEFINITION, "evaluation": EVALUATION, "frame": {"rows": 160, "tags": 4, "seed": 5},
+               "model_build_metadata_keys": tree, "anomaly_columns": [list(c) for c in anomaly.columns],
+               "expanded": _jsonable(expanded), "model_offset": mb["model_offset"], "model_meta": _jsonable(mb["model_meta"]),
+               "scores": _jsonable(mb["cross_validation"]["scores"]), "splits": _jsonable(mb["cross_validation"]["splits"])}
+    with open(os.path.join(HERE, "dropin.json"), "w") as f:
+        json.dump(fixture, f, indent=1, sort_keys=True)
+    arrays = {f"frame_{top}": np.asarray(anomaly[top], dtype=np.float64)
+              for top in dict.fromkeys(anomaly.columns.get_level_values(0)) if top not in ("start", "end")}
+    np.savez_compressed(os.path.join(HERE, "dropin.npz"), **arrays)
+    print("dropin ok", anomaly.shape)
+
+
 if __name__ == "__main__":
     dims_fixture()
     kfcv_fixture("kfcv_smm", 300, 3, 12, "smm", 0.99, seed=6)
@@ -312,3 +389,6 @@ if __name__ == "__main__":
     anomaly_fixture("ffnet_anomaly", 400, 8, None, None, True, base="net", seed=4)
     anomaly_fixture("ffnet_anomaly_t64", 200, 64, None, None, True, base="net", seed=5)
     callers_fixture()
+    for s in (11, 12):
+        detector_fixture(s)
+    dropin_fixture()

@@ -184,9 +184,9 @@ def test_fleet_model_builder_end_to_end(engine, torch, tmp_path):
 
 def test_dropin_definition_on_the_gpu(engine, torch):
     """
-    tests/test_reference_dropin.py runs the INTEGRATION.md definition through the REFERENCE'S from_definition / ModelBuilder._build /
-    serializer.dumps+loads (possible only where /root/reference exists, with the kernels mocked by the oracle) and commits the metadata
-    key tree and the anomaly frame's columns it produced (tests/golden/dropin.json).  Here the same definition and data run on the
+    tests/golden/make_golden.py runs the INTEGRATION.md definition through the REFERENCE'S from_definition / ModelBuilder._build /
+    serializer.dumps+loads (with the kernels mocked by the oracle) and commits the metadata key tree and the anomaly frame's columns
+    it produced (tests/golden/dropin.json).  Here the same definition and data run on the
     real kernels -- per machine (`ModelBuilder`) and through the batched fleet path -- and must produce the same tree and columns.
     """
     import pickle

@@ -1,7 +1,6 @@
 """
 Pins the CPU oracle (oracle/) against (1) fixtures produced by the reference's own code
-(tests/golden/make_golden.py), (2) the golden tables/batches the reference's tests hold,
-(3) the live reference when /root/reference is present (build container only).
+(tests/golden/make_golden.py), (2) the golden tables/batches the reference's tests hold.
 """
 import glob
 import json
@@ -13,7 +12,6 @@ import pytest
 
 from oracle import anomaly_math as am
 from oracle import keras_math as km
-from oracle.reference_loader import reference_available
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 ANOMALY_CASES = sorted(os.path.basename(p)[:-4] for p in glob.glob(os.path.join(GOLDEN, "*anomaly*.npz")))
@@ -163,29 +161,21 @@ def test_base_frame_layout():
     np.testing.assert_array_equal(f["model-input"].values, X[-3:])
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference only exists in the build container")
 @pytest.mark.parametrize("seed", [11, 12])
 def test_live_reference_agrees_with_oracle(seed):
-    from sklearn.linear_model import LinearRegression
-    from sklearn.multioutput import MultiOutputRegressor
-    from sklearn.preprocessing import MinMaxScaler
-
-    from oracle.reference_loader import load_reference
-
-    ref = load_reference()
+    """The reference's DiffBasedAnomalyDetector, cross-validated and fitted on these frames by tests/golden/make_golden.py: its
+    predictions and thresholds through the oracle give its anomaly frame."""
+    g = np.load(os.path.join(GOLDEN, f"detector_sma_seed{seed}.npz"), allow_pickle=False)
     rng = np.random.default_rng(seed)
-    X = pd.DataFrame(rng.random((240, 5)))
-    y = pd.DataFrame(rng.random((240, 5)) * 3.0)
-    det = ref.DiffBasedAnomalyDetector(base_estimator=MultiOutputRegressor(LinearRegression()), scaler=MinMaxScaler(), window=10, smoothing_method="sma")
-    det.cross_validate(X=X, y=y)
-    det.fit(X, y)
-    frame = det.anomaly(X, y)
-    sc, mn = am.minmax_fit(y.values)
-    out = am.anomaly_arrays(det.predict(X), y.values, sc, mn, det.feature_thresholds_.values, det.aggregate_threshold_, 10, "sma")
+    X, y = rng.random((240, 5)), rng.random((240, 5)) * 3.0
+    np.testing.assert_array_equal(g["X"], X)
+    np.testing.assert_array_equal(g["y"], y)
+    sc, mn = am.minmax_fit(y)
+    out = am.anomaly_arrays(g["pred"], y, sc, mn, g["feature_thresholds"], float(g["aggregate_threshold"]), int(g["window"]), str(g["method"]))
     for k, v in out.items():
-        want = frame[k].values
+        want = g[f"frame_{k}"]
         np.testing.assert_allclose(v, want.reshape(v.shape), rtol=1e-9, atol=1e-12, equal_nan=True, err_msg=k)
-    assert tuple(ref.hourglass_calc_dims(0.5, 3, 64)) == km.hourglass_calc_dims(0.5, 3, 64) == (53, 43, 32)
+    assert tuple(g["hourglass_dims_0p5_3_64"]) == km.hourglass_calc_dims(0.5, 3, 64) == (53, 43, 32)
 
 
 def test_ff_fit_reduces_loss_and_history_contract():
